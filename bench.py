@@ -150,6 +150,19 @@ def port_cpu_arm(K, steps, warmup):
             "tasks": dag.ntasks, "steps": len(times), "kind": "port", "sample": "%d groups per step, oracle/orc_cpu_sched.c" % K}
 
 
+def cpu_baseline_arm(K, steps, warmup):
+    """The reference's CPU run where oracle/_ref has one that runs, else the oracle's port.  A reference application
+    that is there but cannot run (a library missing from a copied install, say) is reported, not fatal: the CPU
+    baseline is a record beside the GPU measurement, which must still print its result."""
+    try:
+        r = reference_cpu_arm(K, steps, warmup)
+    except RuntimeError as exc:
+        print("bench.py: the reference's CPU run failed, using the oracle's port: %r" % (exc,), file=sys.stderr)
+        r = port_cpu_arm(K, steps, warmup)
+        r["sample"] += "; the reference's run failed: %s" % str(exc)[:300]
+    return r or port_cpu_arm(K, steps, warmup)
+
+
 def e2e_mca(K, ngpus, steps, cores):
     """e2e through the reference-facing plug-in: reference runtime + parsec/mca/device/b200, host buffers."""
     env = {"PARSEC_MCA_device_b200_enabled": str(ngpus),
@@ -404,6 +417,24 @@ def secondary_cholesky(rank, world, local, torch, dist):
                        "note": "values and versions of this DAG are checked against the oracle at NT=3/8 in the `cholesky` parity case"}}
 
 
+DUMP_TILES = 32
+
+
+def dump_outputs(path, eng, w, slab, K):
+    """What the last timed step of `value` computed, as a caller of the window receives it: per-task results and flow
+    versions, the tiles' final versions, and the data of DUMP_TILES tiles picked by a fixed seed (about 17 MB in all).
+    The retire order, sequence stamps and worker ids depend on scheduling and are left out."""
+    os.makedirs(path, exist_ok=True)
+    res = w.results()
+    pick = np.sort(np.random.default_rng(0).choice(K, size=min(K, DUMP_TILES), replace=False))
+    data = np.empty((len(pick), TILE // 4), np.int32)
+    for row, k in zip(data, pick):                                # slab position k holds tile k of the collection
+        eng.d2h(row, slab + int(k) * TILE)
+    for name, a in (("task_result", res["result"]), ("task_seen_version", res["seen_version"]),
+                    ("tile_version", res["tiles"]["version"]), ("tile_sample_index", pick), ("tile_sample_data", data)):
+        np.save(os.path.join(path, name + ".npy"), a.astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -418,7 +449,11 @@ def main():
     ap.add_argument("--kp", type=int, default=1, help="N>1: k-cyclic factor of the 1xN collection (1: the map of examples/Ex05_Broadcast)")
     ap.add_argument("--mgpu", default="direct", choices=["direct", "exchange"],
                     help="N>1: device-released cross-GPU edges (default) or two windows + one NCCL exchange")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (one GPU only)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs --impl ours on one GPU")
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -440,7 +475,7 @@ def main():
         steps = min(args.steps, max(3, 20 // max(args.gpus, 1)))
         Kref = K * max(args.gpus, 1)
         cfg["reference_workload"] = "%d groups (%d tasks) per step: the whole job of the %d-GPU arm" % (Kref, Kref * (1 + F), max(args.gpus, 1))
-        r = reference_cpu_arm(Kref, steps, args.warmup) or port_cpu_arm(Kref, steps, args.warmup)
+        r = cpu_baseline_arm(Kref, steps, args.warmup)
         print(json.dumps({"impl": "reference", "metric": "tasks/s", "value": r["value"], "unit": "tasks/s", "n_gpus": args.gpus,
                           "steps": r["steps"], "warmup": args.warmup, "ms_per_step": r["ms_per_step"], "higher_is_better": True,
                           "scaling": "weak", "vs_baseline": None, "dtype": "i32", "data": "synthetic", "config": cfg,
@@ -608,6 +643,8 @@ def main():
         st = w.stats
         assert st["body_errors"] == 0 and st["tasks_retired"] == ntasks
         only_kernel_ms = st["kernel_ms"]
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, eng, w, slab, K)
     else:
         dev_ms = ev0.elapsed_time(ev1)                             # engine work is enqueued on torch's current stream
         try:
@@ -639,7 +676,7 @@ def main():
                            "dram_frac": (traffic / (only_kernel_ms / 1e3) / 1e9 / peak) if traffic else None,
                            "l2_frac": (ach / l2_peak) if l2_peak else None, "l2_peak": l2_peak,
                            "note": "frac is ALGORITHMIC bytes (K*(1+F)*262144) over the HBM copy peak and exceeds 1 because 7 of 8 reads of a tile hit the 126 MB L2; dram_frac is the ncu-measured DRAM traffic of the same launch over the same peak; l2_frac is the algorithmic rate over the L2 read rate tools/l2_probe measured on this GPU type"}
-        base = reference_cpu_arm(K, 3, 1) or port_cpu_arm(K, 3, 1)
+        base = cpu_baseline_arm(K, 3, 1)
         out["cpu_baseline"] = {"value": base["value"], "unit": "tasks/s", "cores": base["cores"], "kind": base["kind"], "sample": base["sample"]}
         if not args.no_secondary:
             try:

@@ -12,7 +12,8 @@
 set -e
 ROOT=$(cd "$(dirname "$0")/.." && pwd)
 REF=${REF:-/root/reference}
-SCRATCH=${SCRATCH:-/tmp/pb2_ref}
+# one scratch tree per user and checkout: its CMake cache holds this checkout's paths (PB2_ROOT, the install prefix)
+SCRATCH=${SCRATCH:-${TMPDIR:-/tmp}/pb2_ref-$(id -u)-$(printf %s "$ROOT" | md5sum | cut -c1-12)}
 PREFIX=$ROOT/oracle/_ref/parsec
 [ -d "$REF/parsec" ] || { echo "no reference tree at $REF: keeping the prebuilt oracle/_ref"; exit 0; }
 [ -f "$ROOT/parsec_b200/libparsec_b200.so" ] || { echo "build parsec_b200/libparsec_b200.so first (make)"; exit 1; }
@@ -31,7 +32,7 @@ if [ ! -f "$SCRATCH/build/build.ninja" ] || [ "$1" = "--reconfigure" ]; then
     -DCMAKE_CUDA_COMPILER=/usr/local/cuda/bin/nvcc -DCUDAToolkit_ROOT=/usr/local/cuda \
     -DHWLOC_ROOT="$SCRATCH/hwloc" -DCMAKE_PREFIX_PATH="$SCRATCH/hwloc" \
     -DPB2_ROOT="$ROOT" -DCMAKE_INSTALL_PREFIX="$PREFIX" \
-    -DCMAKE_INSTALL_RPATH='$ORIGIN;$ORIGIN/../../../../parsec_b200' -DCMAKE_BUILD_WITH_INSTALL_RPATH=ON > "$SCRATCH/configure.log" 2>&1 \
+    -DCMAKE_PROJECT_PARSEC_INCLUDE="$ROOT/oracle/ref_rpath.cmake" > "$SCRATCH/configure.log" 2>&1 \
     || { tail -30 "$SCRATCH/configure.log"; exit 1; }
   grep -E "Module .b200|Active modules for the device" "$SCRATCH/configure.log" || true
 fi
@@ -40,4 +41,9 @@ rm -rf "$PREFIX"
 cmake --install "$SCRATCH/build" > "$SCRATCH/install.log" 2>&1 || { tail -20 "$SCRATCH/install.log"; exit 1; }
 # the shim's header is needed by whoever includes parsec's devel headers
 cp "$ROOT/oracle/hwloc_shim/hwloc.h" "$PREFIX/include/"
+# the install travels to other machines by copies that may drop symbolic links (libparsec.so.4 -> libparsec.so.4.1.0,
+# the name the applications load): turn every link into a copy of its target
+find "$PREFIX" -type l | while read -r l; do t=$(readlink -f "$l"); rm "$l"; cp "$t" "$l"; done
+# and for the same reason the RUNPATH of libparsec (ref_rpath.cmake) must not name this checkout
+if readelf -d "$PREFIX/lib/libparsec.so" | grep -F "$ROOT"; then echo "libparsec.so has an absolute RUNPATH: run $0 --reconfigure"; exit 1; fi
 du -sh "$PREFIX" | sed 's/^/installed: /'
