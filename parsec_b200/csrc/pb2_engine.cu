@@ -52,10 +52,7 @@ __global__ void pb2_window_reset_kernel(WinDev w, const pb2_tile_t* tiles_init,
         w.ring[i] = (i < (size_t)nready) ? ready[i] : kEmpty;
     for (size_t i = gid; i < (size_t)w.ntiles; i += gsz) {
         w.tiles[i] = tiles_init[i];
-        if (w.slice_claim) {
-            for (int k = 0; k < PB2_SLICE_WORDS; ++k) w.slice_claim[i * PB2_SLICE_WORDS + k] = 0;
-            for (int k = 0; k <= PB2_SLICE_WORDS; ++k) w.slice_done[i * (PB2_SLICE_WORDS + 1) + k] = 0;
-        }
+        if (w.slice_claim) reset_tile_slices(w, i);
     }
     if (gid == 0) {
         w.ctl->head.v = 0; w.ctl->tail.v = (unsigned long long)nready; w.ctl->evt.v = 0;
@@ -119,11 +116,7 @@ pb2_engine_hbm_kernel(WinDev w) {
                 if (nparts > 1) { last = atomicSub(&w.parts_left[id], 1) == 1; __threadfence(); }
                 s.window_done = 0; s.last = last;
                 if (last) {
-                    epilog_written_flows(w, t);
-                    w.end_seq[id] = (uint32_t)atomicAdd(&w.ctl->evt.v, 1ull);
-                    // the retire log is written before the out-edges are released, so that it is a linear
-                    // extension of the DAG's partial order (a successor can only retire after us)
-                    s.window_done = retire_task(w, id) ? 1 : 0;
+                    s.window_done = retire_task(w, t, id) ? 1 : 0;
                     __threadfence();
                 }
             }
@@ -136,10 +129,7 @@ pb2_engine_hbm_kernel(WinDev w) {
         }
         if (threadIdx.x < 32) {
             if (s.last) { release_successors_warp(w, s.task); release_remote_warp(w, id); }
-            if (threadIdx.x == 0 && s.window_done) {
-                __threadfence();
-                st_release_gpu(reinterpret_cast<int32_t*>(&w.ctl->done.v), kDoneOK);
-            }
+            if (threadIdx.x == 0 && s.window_done) finish_window(w);
         }
         __syncthreads();
     }
@@ -723,7 +713,7 @@ int pb2_window_create(pb2_engine_t* e, pb2_window_t** window, int kind,
     w->shared = e->shared_windows;
     w->e = e; w->kind = kind; w->ntasks = ntasks; w->nsucc = nsucc; w->ntiles = ntiles; w->nready = nready;
 #define TRY(x) do { rc = (x); if (rc != PB2_SUCCESS) { pb2_window_destroy(w); return rc; } } while (0)
-    // wide tasks (HBM windows): parts per task = ceil(widest tile / part_bytes), at most PB2_MAX_PARTS
+    // wide tasks (HBM windows): the parts of a task are the tile_parts of its widest tile
     std::vector<pb2_task_t> dtasks(tasks, tasks + ntasks);
     std::vector<uint16_t> nparts((size_t)ntasks, 1);
     std::vector<int32_t> entries;
@@ -734,9 +724,8 @@ int pb2_window_create(pb2_engine_t* e, pb2_window_t** window, int kind,
         if (kind != 0 || t.body == PB2_BODY_NOP || e->params.part_bytes < 0 || ntasks >= (1 << 22)) continue;
         uint32_t big = 0;
         for (int f = 0; f < t.nb_flows; ++f) if (t.tile[f] >= 0 && tiles[t.tile[f]].bytes > big) big = tiles[t.tile[f]].bytes;
-        uint32_t np = (big + (uint32_t)e->params.part_bytes - 1) / (uint32_t)e->params.part_bytes;
-        if (np > PB2_MAX_PARTS) np = PB2_MAX_PARTS;
-        if (np > 1) { nparts[(size_t)i] = (uint16_t)np; extra_parts += np - 1; }
+        const int np = tile_parts(big, e->params.part_bytes);
+        if (np > 1) { nparts[(size_t)i] = (uint16_t)np; extra_parts += (uint32_t)np - 1; }
     }
     for (int32_t i = 0; i < nready; ++i)
         for (int p = 0; p < (int)nparts[(size_t)ready[i]]; ++p) entries.push_back(PB2_ENT_MAKE(ready[i], p));

@@ -16,7 +16,7 @@
 // 128B-swizzled boxes filled by TMA (`cp.async.bulk.tensor.2d`) from per-tile tensor maps.
 #pragma once
 #include <cuda.h>
-#include "pb2_sched.cuh"
+#include "pb2_worker.cuh"
 
 namespace pb2 {
 
@@ -177,8 +177,7 @@ pb2_engine_gemm_kernel(WinDev w, const CUtensorMap* __restrict__ tmaps) {
         if (threadIdx.x == 0) {
             int need = 0;
             for (int f = 0; f < t.nb_flows; ++f)
-                if (t.tile[f] >= 0 && (t.access[f] & PB2_FLOW_ACCESS_READ) &&
-                    ld_acquire_gpu(&w.tiles[t.tile[f]].state) != PB2_TILE_VALID) need |= 1 << f;
+                if (t.tile[f] >= 0 && needs_stage_in(&w.tiles[t.tile[f]], t.access[f])) need |= 1 << f;
             sh.need = need;
         }
         __syncthreads();
@@ -306,38 +305,22 @@ pb2_engine_gemm_kernel(WinDev w, const CUtensorMap* __restrict__ tmaps) {
 
         // ---- pushout (PARSEC_PUSHOUT on the last k, dtd_test_simple_gemm.c:687) ----
         for (int f = 0; f < t.nb_flows; ++f) {
-            if (t.tile[f] >= 0 && (t.access[f] & PB2_FLOW_PUSHOUT) && (t.access[f] & PB2_FLOW_ACCESS_WRITE)) {
-                pb2_tile_t* tile = &w.tiles[t.tile[f]];
-                cta_copy<false>(tile->src_ptr, tile->dev_ptr, tile->bytes);
-                if (threadIdx.x == 0) atomicAdd(&w.ctl->bytes_d2h.v, (unsigned long long)tile->bytes);
-            }
+            if (pushes_out(t, f)) pushout(w.ctl, w.tiles[t.tile[f]].src_ptr, w.tiles[t.tile[f]].dev_ptr, w.tiles[t.tile[f]].bytes);
         }
         __syncthreads();
 
         if (threadIdx.x < 32) {
             __threadfence();
             if (threadIdx.x == 0) {
-                w.result[id] = hbm_result;
-                if ((t.body == PB2_BODY_CHECK_I32 || t.body == PB2_BODY_CHECK_F32) && (hbm_result >> 32))
-                    atomicAdd(&w.ctl->body_errors.v, hbm_result >> 32);
-                for (int f = 0; f < t.nb_flows; ++f) {
-                    if (t.tile[f] < 0 || !(t.access[f] & PB2_FLOW_ACCESS_WRITE)) continue;
-                    pb2_tile_t* tile = &w.tiles[t.tile[f]];
-                    *reinterpret_cast<volatile uint32_t*>(&tile->version) =
-                        *reinterpret_cast<volatile uint32_t*>(&tile->version) + 1;
-                    if (!(t.access[f] & PB2_FLOW_ACCESS_READ)) st_relaxed_gpu(&tile->state, PB2_TILE_VALID);
-                }
-                w.end_seq[id] = (uint32_t)atomicAdd(&w.ctl->evt.v, 1ull);
-                sh.last = retire_task(w, id) ? 1 : 0;
+                // a body id validate_window accepts but run_hbm_body does not know (result ~0) does not abort here
+                record_result(w, t.body, id, 0, 1, hbm_result);
+                sh.last = retire_task(w, t, id) ? 1 : 0;
                 __threadfence();
             }
             __syncwarp();
             release_successors_warp(w, t);
             release_remote_warp(w, id);
-            if (threadIdx.x == 0 && sh.last) {
-                __threadfence();
-                st_release_gpu(reinterpret_cast<int32_t*>(&w.ctl->done.v), kDoneOK);
-            }
+            if (threadIdx.x == 0 && sh.last) finish_window(w);
         }
         __syncthreads();
     }

@@ -14,7 +14,7 @@
 //   * scheduling entities on the device are units (counter-mode dependency words), ring entries are (part, unit).
 #pragma once
 #include <cuda.h>
-#include "pb2_sched.cuh"
+#include "pb2_worker.cuh"
 #include "pb2_gemm.cuh"
 
 namespace pb2 {
@@ -106,9 +106,6 @@ __device__ __forceinline__ void tc_commit2(uint64_t* bar) {
                  :: "r"(smem_u32(bar)), "h"((uint16_t)0x3) : "memory");
 }
 
-// one thread: pop a (part, unit) entry; same ticket ring as the task-level kernels
-__device__ __forceinline__ int32_t pop_entry(const WinDev& w) { return pop_task(w); }
-
 // whole warp: the unit is complete (all parts): retire its members in chain order, release its out-edges
 __device__ __forceinline__ void retire_unit_warp(const Win2Dev& g, const GUnit& u, int unit_id) {
     const WinDev& w = g.w;
@@ -162,25 +159,12 @@ __device__ __forceinline__ void retire_unit_warp(const Win2Dev& g, const GUnit& 
             sid = g.usucc[u.succ_begin + e];
             if (atomicSub(&g.udep[sid], 1) == 1) nparts = g.units[sid].nparts;
         }
-        // exclusive scan of nparts over the warp
-        int incl = nparts;
-        for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += v; }
-        const int total = __shfl_sync(0xffffffffu, incl, 31);
-        if (total) {
-            unsigned long long base = 0;
-            if (lane == 0) base = atomicAdd(&w.ctl->tail.v, (unsigned long long)total);
-            base = __shfl_sync(0xffffffffu, base, 0);
-            for (int p = 0; p < nparts; ++p)
-                st_release_gpu(&w.ring[((uint32_t)base + (uint32_t)(incl - nparts + p)) & w.cap_mask], (int32_t)PB2_SUCC_MAKE(sid, p));
-        }
+        push_ready_warp<true>(w, sid, nparts);
     }
     // out-edges into other GPUs' windows, member by member (a member with remote successors is always the last of
     // its unit: build_gemm2_units does not fuse across it)
     if (w.rs_begin) for (int i = 0; i < L; ++i) release_remote_warp(w, g.segs[u.seg_begin + i].task);
-    if (lane == 0 && (int32_t)(rbase + L) == w.ntasks) {
-        __threadfence();
-        st_release_gpu(reinterpret_cast<int32_t*>(&w.ctl->done.v), kDoneOK);
-    }
+    if (lane == 0 && (int32_t)(rbase + L) == w.ntasks) finish_window(w);
     (void)unit_id;
 }
 
@@ -220,7 +204,7 @@ pb2_engine_gemm2_kernel(Win2Dev g) {
         if (leader) {
             if (threadIdx.x == 0) {
                 Job j; memset(&j, 0, sizeof j);
-                const int32_t e = pop_entry(w);
+                const int32_t e = pop_task(w);
                 if (e == kEmpty) { j.stop = 1; }
                 else {
                     __threadfence();
@@ -243,7 +227,7 @@ pb2_engine_gemm2_kernel(Win2Dev g) {
                     if (i < 0) { if (!sh.job.is_gemm) break; tile_id = sh.job.tileC; acc = PB2_FLOW_ACCESS_RW; }
                     else { const GSeg s = g.segs[sh.job.seg_begin + (i >> 1)]; tile_id = (i & 1) ? s.tileB : s.tileA; acc = PB2_FLOW_ACCESS_READ; }
                     pb2_tile_t* tile = &w.tiles[tile_id];
-                    if (threadIdx.x == 0) sh.need = ld_acquire_gpu(&tile->state) != PB2_TILE_VALID;
+                    if (threadIdx.x == 0) sh.need = needs_stage_in(tile, acc);
                     __syncthreads();
                     if (sh.need) {
                         const int ns = tile_slices(w, tile->bytes);
@@ -262,7 +246,7 @@ pb2_engine_gemm2_kernel(Win2Dev g) {
                     for (int f = 0; f < t.nb_flows; ++f) {
                         if (t.tile[f] < 0 || !(t.access[f] & PB2_FLOW_ACCESS_READ)) continue;
                         pb2_tile_t* tile = &w.tiles[t.tile[f]];
-                        if (threadIdx.x == 0) sh.need = ld_acquire_gpu(&tile->state) != PB2_TILE_VALID;
+                        if (threadIdx.x == 0) sh.need = needs_stage_in(tile, t.access[f]);
                         __syncthreads();
                         if (sh.need) { stage_in_flow(stage_ctx(w), tile, t.access[f], &sh.decide); fence_proxy_async(); }
                         __syncthreads();
@@ -406,17 +390,11 @@ pb2_engine_gemm2_kernel(Win2Dev g) {
             a.elem0 = 0; a.part = 0;
             a.iparam[0] = t.iparam[0]; a.iparam[1] = t.iparam[1]; a.iparam[2] = t.iparam[2]; a.fparam = t.fparam;
             const unsigned long long r = run_hbm_body(t.body, a, sh.red);
-            if (threadIdx.x == 0) {
-                w.result[g.segs[job.seg_begin].task] = r;
-                if ((t.body == PB2_BODY_CHECK_I32 || t.body == PB2_BODY_CHECK_F32) && (r >> 32)) atomicAdd(&w.ctl->body_errors.v, r >> 32);
-            }
+            // as in the v1 kernel, an unknown body id does not abort the window
+            if (threadIdx.x == 0) record_result(w, t.body, g.segs[job.seg_begin].task, 0, 1, r);
             fence_proxy_async();
             for (int f = 0; f < t.nb_flows; ++f)
-                if (t.tile[f] >= 0 && (t.access[f] & PB2_FLOW_PUSHOUT) && (t.access[f] & PB2_FLOW_ACCESS_WRITE)) {
-                    pb2_tile_t* tile = &w.tiles[t.tile[f]];
-                    cta_copy<false>(tile->src_ptr, tile->dev_ptr, tile->bytes);
-                    if (threadIdx.x == 0) atomicAdd(&w.ctl->bytes_d2h.v, (unsigned long long)tile->bytes);
-                }
+                if (pushes_out(t, f)) pushout(w.ctl, w.tiles[t.tile[f]].src_ptr, w.tiles[t.tile[f]].dev_ptr, w.tiles[t.tile[f]].bytes);
         }
         __threadfence();
         cluster_sync_all();          // every store of the part (both CTAs) is done and visible
@@ -428,9 +406,8 @@ pb2_engine_gemm2_kernel(Win2Dev g) {
                 const size_t row_bytes = (size_t)job.N * 2;
                 const int rows = min(256, job.M - job.m0);
                 if (rows > 0 && job.Nj == job.N) {
-                    cta_copy<false>(reinterpret_cast<uint8_t*>(tile->src_ptr) + (size_t)job.m0 * row_bytes,
-                                    reinterpret_cast<const uint8_t*>(tile->dev_ptr) + (size_t)job.m0 * row_bytes, (size_t)rows * row_bytes);
-                    if (threadIdx.x == 0) atomicAdd(&w.ctl->bytes_d2h.v, (unsigned long long)rows * row_bytes);
+                    pushout(w.ctl, reinterpret_cast<uint8_t*>(tile->src_ptr) + (size_t)job.m0 * row_bytes,
+                            reinterpret_cast<const uint8_t*>(tile->dev_ptr) + (size_t)job.m0 * row_bytes, (size_t)rows * row_bytes);
                 } else if (rows > 0) {
                     // a column block of a tile wider than 512: row segments
                     for (int r = 0; r < rows; ++r) {

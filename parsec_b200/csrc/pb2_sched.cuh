@@ -68,32 +68,55 @@ struct alignas(32) PushDev { void* dst; int32_t* dst_state; uint32_t bytes; int3
 // the machine, not 1 ms of one CTA).  Parts per task (1..512) live in WinDev::nparts; ring entries of HBM windows
 // are (part << 22) | task, so such a window holds at most 2^22 tasks when it has wide tasks.
 #define PB2_MAX_PARTS 512
+#define PB2_SLICE_WORDS (PB2_MAX_PARTS / 32)
 #define PB2_ENT_MAKE(task, part) ((int32_t)(((uint32_t)(part) << 22) | (uint32_t)(task)))
 #define PB2_ENT_TASK(e)          ((int32_t)((uint32_t)(e) & 0x3FFFFFu))
 #define PB2_ENT_PART(e)          ((int)((uint32_t)(e) >> 22))
 
+// Parts of a tile cut at part_bytes (> 0): the parts of a wide task (its widest tile) and the stage-in slices of a tile.
+__host__ __device__ __forceinline__ int tile_parts(uint32_t bytes, int32_t part_bytes) {
+    const uint32_t n = (bytes + (uint32_t)part_bytes - 1) / (uint32_t)part_bytes;
+    return n > PB2_MAX_PARTS ? PB2_MAX_PARTS : (n < 1 ? 1 : (int)n);
+}
+
+// Slice i of n slices of `per` = slice_size bytes: [off, off + len); the last one takes the remainder.
+__host__ __device__ __forceinline__ uint32_t slice_size(uint32_t bytes, int n) { return ((bytes / (uint32_t)n) + 15u) & ~15u; }
+__host__ __device__ __forceinline__ void slice_bounds(uint32_t per, uint32_t bytes, int i, int n, uint32_t& off, uint32_t& len) {
+    off = per * (uint32_t)i < bytes ? per * (uint32_t)i : bytes;
+    len = (i == n - 1) ? bytes - off : (off + per <= bytes ? per : bytes - off);
+}
+
+// Stamp of index idx of a ring of `slots` entries (never 0).
+__host__ __device__ __forceinline__ uint32_t ring_gen(unsigned long long idx, unsigned long long slots) {
+    return (uint32_t)(idx / slots) + 1u;
+}
+
 __device__ __forceinline__ int task_nparts(const WinDev& w, int32_t id) { return w.nparts ? (int)w.nparts[id] : 1; }
 
-// Whole warp: lanes with np > 0 own a ready task `sid` whose entries go to ring[first .. first + np).  Tasks with
-// hundreds of parts are written by all 32 lanes together.
-template <bool SYS>
-__device__ __forceinline__ void push_entries_warp(int32_t* ring, uint32_t cap_mask, int32_t sid, int np, uint32_t first) {
+// Whole warp: a lane with np > 0 pushes the entries of parts 0 .. np-1 of ready `sid`, one tail reservation per warp.
+// UNITS: v2 GEMM units (PB2_SUCC_MAKE, <= 16 parts), written lane by lane: fewer registers in pb2_engine_gemm2_kernel.
+template <bool UNITS>
+__device__ __forceinline__ void push_ready_warp(const WinDev& w, int32_t sid, int np) {
     const int lane = threadIdx.x & 31;
-    const unsigned many = __ballot_sync(0xffffffffu, np > 4);
-    if (np > 0 && np <= 4)
-        for (int p = 0; p < np; ++p) {
-            if (SYS) st_release_sys(&ring[(first + (uint32_t)p) & cap_mask], PB2_ENT_MAKE(sid, p));
-            else st_release_gpu(&ring[(first + (uint32_t)p) & cap_mask], PB2_ENT_MAKE(sid, p));
-        }
+    int incl = np;
+    for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += v; }
+    const int total = __shfl_sync(0xffffffffu, incl, 31);
+    if (!total) return;
+    unsigned long long base = 0;
+    if (lane == 0) base = atomicAdd(&w.ctl->tail.v, (unsigned long long)total);
+    base = __shfl_sync(0xffffffffu, base, 0);
+    const uint32_t first = (uint32_t)base + (uint32_t)(incl - np);
+    const unsigned many = UNITS ? 0u : __ballot_sync(0xffffffffu, np > 4);
+    if (np > 0 && (UNITS || np <= 4))
+        for (int p = 0; p < np; ++p)
+            st_release_gpu(&w.ring[(first + (uint32_t)p) & w.cap_mask], UNITS ? (int32_t)PB2_SUCC_MAKE(sid, p) : PB2_ENT_MAKE(sid, p));
     for (unsigned m = many; m; m &= m - 1) {
         const int src = __ffs(m) - 1;
         const int32_t s2 = __shfl_sync(0xffffffffu, sid, src);
         const int n2 = __shfl_sync(0xffffffffu, np, src);
         const uint32_t f2 = __shfl_sync(0xffffffffu, first, src);
-        for (int p = lane; p < n2; p += 32) {
-            if (SYS) st_release_sys(&ring[(f2 + (uint32_t)p) & cap_mask], PB2_ENT_MAKE(s2, p));
-            else st_release_gpu(&ring[(f2 + (uint32_t)p) & cap_mask], PB2_ENT_MAKE(s2, p));
-        }
+        for (int p = lane; p < n2; p += 32)
+            st_release_gpu(&w.ring[(f2 + (uint32_t)p) & w.cap_mask], UNITS ? (int32_t)PB2_SUCC_MAKE(s2, p) : PB2_ENT_MAKE(s2, p));
     }
 }
 
@@ -108,11 +131,7 @@ __device__ __forceinline__ int32_t pop_task(const WinDev& w) {
     int32_t* slot = &w.ring[ticket & w.cap_mask];
     uint32_t spins = 0;
     int32_t id;
-#ifdef PB2_EXPERIMENT_GPU_SCOPE_POLL
-    while ((id = ld_acquire_gpu(slot)) == kEmpty) {
-#else
     while ((id = (w.shared ? ld_acquire_sys(slot) : ld_acquire_gpu(slot))) == kEmpty) {
-#endif
         if (ld_relaxed_gpu(reinterpret_cast<const int32_t*>(&w.ctl->done.v)) != 0) return kEmpty;
         if ((++spins & 1023u) == 0) {
             // watchdog: a DAG whose dependency counts are wrong would spin forever
@@ -151,17 +170,7 @@ __device__ __forceinline__ void release_successors_warp(const WinDev& w, const p
                 ready = (atomicSub(&w.dep[sid], 1) == 1);
             }
         }
-        // a ready successor contributes one ring entry per part: exclusive scan of the part counts over the warp
-        const int nparts = ready ? task_nparts(w, sid) : 0;
-        int incl = nparts;
-        for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += v; }
-        const int total = __shfl_sync(0xffffffffu, incl, 31);
-        if (total) {
-            unsigned long long base = 0;
-            if (lane == 0) base = atomicAdd(&w.ctl->tail.v, (unsigned long long)total);
-            base = __shfl_sync(0xffffffffu, base, 0);
-            push_entries_warp<false>(w.ring, w.cap_mask, sid, nparts, (uint32_t)base + (uint32_t)(incl - nparts));
-        }
+        push_ready_warp<false>(w, sid, ready ? task_nparts(w, sid) : 0);
     }
 }
 
@@ -225,12 +234,15 @@ static __device__ __noinline__ void push_written_tiles(const pb2_tile_t* tiles, 
     __syncthreads();
 }
 
-// One thread: append to the retire log; returns true when this was the last task of the window.
-__device__ __forceinline__ bool retire_task(const WinDev& w, int32_t id) {
-    const uint32_t seq = (uint32_t)atomicAdd(&w.ctl->retired.v, 1ull);
-    w.retire_log[seq] = id;
-    *reinterpret_cast<volatile unsigned long long*>(&w.ctl->progress_ns.v) = globaltimer_ns();
-    return (int32_t)(seq + 1) == w.ntasks;
+// One thread, after the window's last task released its out-edges.
+__device__ __forceinline__ void finish_window(const WinDev& w) {
+    __threadfence();
+    st_release_gpu(reinterpret_cast<int32_t*>(&w.ctl->done.v), kDoneOK);
+}
+
+__device__ __forceinline__ void reset_tile_slices(const WinDev& w, size_t tile) {
+    for (int k = 0; k < PB2_SLICE_WORDS; ++k) w.slice_claim[tile * PB2_SLICE_WORDS + k] = 0;
+    for (int k = 0; k <= PB2_SLICE_WORDS; ++k) w.slice_done[tile * (PB2_SLICE_WORDS + 1) + k] = 0;
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -245,22 +257,37 @@ __device__ __forceinline__ StageCtx stage_ctx(const WinDev& w) {
     return StageCtx{w.tiles, w.ctl, w.slice_claim, w.slice_done, w.stage_mode == 0 ? 1 : 0, w.part_bytes};
 }
 
+// parsec_device_data_stage_in, device_gpu.c:1799-2165: only a READ access needs the bytes;
+// "finally we'll just overwrite w/o read" (data.c:427) for WRITE-only flows.
+__device__ __forceinline__ bool needs_stage_in(const pb2_tile_t* tile, uint8_t access) {
+    return (access & PB2_FLOW_ACCESS_READ) && ld_acquire_gpu(&tile->state) != PB2_TILE_VALID;
+}
+
+// One thread: wait for a tile or slice that another worker (SYS: a producer on another GPU) moves.
+template <bool SYS>
+__device__ __forceinline__ void wait_word(const int32_t* word, int32_t mask, int32_t want) {
+    while (((SYS ? ld_acquire_sys(word) : ld_acquire_gpu(word)) & mask) != want) __nanosleep(64);
+}
+
+__device__ __forceinline__ void count_stage_in(Ctl* ctl, const pb2_tile_t* tile, uint32_t bytes) {
+    atomicAdd(tile->src_kind == PB2_SRC_PEER ? &ctl->bytes_d2d.v : &ctl->bytes_h2d.v, (unsigned long long)bytes);
+}
+
 // Thread 0 decides (s_decide[0]): 1 = this CTA moves the tile, 0 = already valid (possibly after waiting)
 static __device__ __noinline__ void stage_in_flow(const StageCtx w, pb2_tile_t* tile, uint8_t access, int* s_decide, BulkSmem* bulk = nullptr) {
     if (threadIdx.x == 0) {
         int decide = 0;
         if ((access & PB2_FLOW_ACCESS_READ) && tile->src_kind == PB2_SRC_PUSH) {
             // the producer writes this slot and publishes its state before it releases us: nothing to move
-            while (ld_acquire_sys(&tile->state) != PB2_TILE_VALID) __nanosleep(64);
+            wait_word<true>(&tile->state, -1, PB2_TILE_VALID);
         } else if (access & PB2_FLOW_ACCESS_READ) {
-            // parsec_device_data_stage_in, device_gpu.c:1799-2165: only a READ access needs the bytes;
-            // "finally we'll just overwrite w/o read" (data.c:427) for WRITE-only flows.
             int32_t st = atomicCAS(&tile->state, PB2_TILE_INVALID, PB2_TILE_STAGING);
             if (st == PB2_TILE_INVALID) {
                 decide = 1;
-            } else {
-                // another worker is moving it: "data copy is already under transfer" (:1873-1884)
-                while (st != PB2_TILE_VALID) { __nanosleep(64); st = ld_acquire_gpu(&tile->state); }
+            } else if (st != PB2_TILE_VALID) {
+                // another worker is moving it: "data copy is already under transfer" (device_gpu.c:1873-1884)
+                __nanosleep(64);
+                wait_word<false>(&tile->state, -1, PB2_TILE_VALID);
             }
         }
         *s_decide = decide;
@@ -271,9 +298,8 @@ static __device__ __noinline__ void stage_in_flow(const StageCtx w, pb2_tile_t* 
         __syncthreads();
         if (threadIdx.x == 0) {
             __threadfence();
-            st_release_gpu(&tile->state, PB2_TILE_VALID);   // COMPLETE_TRANSFER (:2358-2573)
-            atomicAdd(tile->src_kind == PB2_SRC_PEER ? &w.ctl->bytes_d2d.v : &w.ctl->bytes_h2d.v,
-                      (unsigned long long)tile->bytes);
+            st_release_gpu(&tile->state, PB2_TILE_VALID);   // COMPLETE_TRANSFER (device_gpu.c:2358-2573)
+            count_stage_in(w.ctl, tile, tile->bytes);
             atomicAdd(&w.ctl->stage_ins.v, 1ull);
         }
     }
@@ -281,12 +307,10 @@ static __device__ __noinline__ void stage_in_flow(const StageCtx w, pb2_tile_t* 
 }
 
 
-// Number of stage-in slices of a tile: the same rule pb2_window_create uses for the parts of a wide task.
-#define PB2_SLICE_WORDS (PB2_MAX_PARTS / 32)
+// Number of stage-in slices of a tile.
 __device__ __forceinline__ int tile_slices_of(int32_t part_bytes, const uint32_t* slice_claim, uint32_t bytes) {
     if (part_bytes <= 0 || !slice_claim) return 1;
-    const uint32_t n = (bytes + (uint32_t)part_bytes - 1) / (uint32_t)part_bytes;
-    return n > PB2_MAX_PARTS ? PB2_MAX_PARTS : (n < 1 ? 1 : (int)n);
+    return tile_parts(bytes, part_bytes);
 }
 __device__ __forceinline__ int tile_slices(const WinDev& w, uint32_t bytes) { return tile_slices_of(w.part_bytes, w.slice_claim, bytes); }
 
@@ -297,12 +321,12 @@ __device__ __forceinline__ int tile_slices(const WinDev& w, uint32_t bytes) { re
 static __device__ __noinline__ void stage_in_slices(const StageCtx w, int32_t tile_id, int nslices, int s0, int s1, int* s_decide, BulkSmem* bulk = nullptr) {
     pb2_tile_t* tile = &w.tiles[tile_id];
     if (tile->src_kind == PB2_SRC_PUSH) {       // written by its producer (see stage_in_flow)
-        if (threadIdx.x == 0) while (ld_acquire_sys(&tile->state) != PB2_TILE_VALID) __nanosleep(64);
+        if (threadIdx.x == 0) wait_word<true>(&tile->state, -1, PB2_TILE_VALID);
         __syncthreads();
         return;
     }
     const uint32_t bytes = tile->bytes;
-    const uint32_t sper = ((bytes / (uint32_t)nslices) + 15u) & ~15u;
+    const uint32_t sper = slice_size(bytes, nslices);
     uint32_t* claim = w.slice_claim + (size_t)tile_id * PB2_SLICE_WORDS;
     uint32_t* done = w.slice_done + (size_t)tile_id * (PB2_SLICE_WORDS + 1);     // last word: number of staged slices
     for (int sl = s0; sl < s1; ++sl) {
@@ -310,14 +334,14 @@ static __device__ __noinline__ void stage_in_slices(const StageCtx w, int32_t ti
         if (threadIdx.x == 0) *s_decide = (atomicOr(&claim[sl >> 5], bit) & bit) ? 0 : 1;
         __syncthreads();
         if (*s_decide) {
-            const uint32_t off = sper * (uint32_t)sl < bytes ? sper * (uint32_t)sl : bytes;
-            const uint32_t len = (sl == nslices - 1) ? bytes - off : (off + sper <= bytes ? sper : bytes - off);
+            uint32_t off, len;
+            slice_bounds(sper, bytes, sl, nslices, off, len);
             cta_copy<true>(reinterpret_cast<uint8_t*>(tile->dev_ptr) + off, reinterpret_cast<const uint8_t*>(tile->src_ptr) + off, len, w.use_bulk ? bulk : nullptr);
             __syncthreads();
             if (threadIdx.x == 0) {
                 __threadfence();
                 atomicOr(&done[sl >> 5], bit);
-                atomicAdd(tile->src_kind == PB2_SRC_PEER ? &w.ctl->bytes_d2d.v : &w.ctl->bytes_h2d.v, (unsigned long long)len);
+                count_stage_in(w.ctl, tile, len);
                 if ((int)atomicAdd(&done[PB2_SLICE_WORDS], 1u) + 1 == nslices) {
                     __threadfence();
                     st_release_gpu(&tile->state, PB2_TILE_VALID);
@@ -329,8 +353,8 @@ static __device__ __noinline__ void stage_in_slices(const StageCtx w, int32_t ti
     }
     if (threadIdx.x == 0) {
         for (int sl = s0; sl < s1; ++sl) {
-            const uint32_t bit = 1u << (sl & 31);
-            while (!(ld_acquire_gpu(reinterpret_cast<const int32_t*>(&done[sl >> 5])) & bit)) __nanosleep(64);
+            const int32_t bit = (int32_t)(1u << (sl & 31));
+            wait_word<false>(reinterpret_cast<const int32_t*>(&done[sl >> 5]), bit, bit);
         }
         __threadfence();
     }

@@ -135,7 +135,7 @@ __device__ __forceinline__ void dispatcher_warp(const StreamDev& sd) {
         // phase 1: which of the next 32 commands are there?  (stamp == generation of the index, stored last)
         const unsigned long long idx = head + (unsigned long long)lane;
         const Cmd* c = &sd.cmd[idx & sd.cmd_mask];
-        const uint32_t want = (uint32_t)(idx / ((unsigned long long)sd.cmd_mask + 1ull)) + 1u;
+        const uint32_t want = ring_gen(idx, sd.cmd_mask + 1ull);
         const uint32_t got = ld_volatile_u32(&c->stamp);
         const unsigned validm = __ballot_sync(0xffffffffu, got == want);
         const int n = (validm == 0xffffffffu) ? 32 : (__ffs(~validm) - 1);
@@ -150,7 +150,7 @@ __device__ __forceinline__ void dispatcher_warp(const StreamDev& sd) {
                     // is either seen here (we stay) or the host relaunches (it re-reads the state after storing)
                     sd.hctl->state = HS_STOPPED;
                     __threadfence_system();
-                    if (ld_volatile_u32(&sd.cmd[head & sd.cmd_mask].stamp) == (uint32_t)(head / ((unsigned long long)sd.cmd_mask + 1ull)) + 1u) {
+                    if (ld_volatile_u32(&sd.cmd[head & sd.cmd_mask].stamp) == ring_gen(head, sd.cmd_mask + 1ull)) {
                         sd.hctl->state = HS_RUNNING;
                         __threadfence_system();
                     } else leave = 1;
@@ -202,10 +202,7 @@ __device__ __forceinline__ void dispatcher_warp(const StreamDev& sd) {
                 t.src_ptr = reinterpret_cast<void*>(((unsigned long long)q2.y << 32) | q2.x);
                 t.bytes = q2.z;
                 w.tiles[tile] = t;
-                if (w.slice_claim && t.state != PB2_TILE_VALID) {
-                    for (int k = 0; k < PB2_SLICE_WORDS; ++k) w.slice_claim[(size_t)tile * PB2_SLICE_WORDS + k] = 0;
-                    for (int k = 0; k <= PB2_SLICE_WORDS; ++k) w.slice_done[(size_t)tile * (PB2_SLICE_WORDS + 1) + k] = 0;
-                }
+                if (w.slice_claim && t.state != PB2_TILE_VALID) reset_tile_slices(w, (size_t)tile);
             }
         } else if (op == CMD_TASK) {
             ticket = (int32_t)q0.z;
@@ -228,19 +225,8 @@ __device__ __forceinline__ void dispatcher_warp(const StreamDev& sd) {
         }
         __threadfence();
         __syncwarp();
-        // phase B: ready tasks enter the ring in command order (warp scan of their part counts)
-        {
-            const int mine = (op == CMD_TASK && goal == 0) ? np : 0;
-            int incl = mine;
-            for (int o = 1; o < 32; o <<= 1) { const int v = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += v; }
-            const int total = __shfl_sync(0xffffffffu, incl, 31);
-            if (total) {
-                unsigned long long base = 0;
-                if (lane == 0) base = atomicAdd(&w.ctl->tail.v, (unsigned long long)total);
-                base = __shfl_sync(0xffffffffu, base, 0);
-                push_entries_warp<false>(w.ring, w.cap_mask, ticket, mine, (uint32_t)base + (uint32_t)(incl - mine));
-            }
-        }
+        // phase B: ready tasks enter the ring in command order
+        push_ready_warp<false>(w, ticket, (op == CMD_TASK && goal == 0) ? np : 0);
         // phase C: look-ahead edges.  A predecessor that has already closed its list counts as satisfied.
         if (op == CMD_EDGE) {
             const int32_t pred = (int32_t)q0.z, succ = (int32_t)q0.w, node = (int32_t)q1.x;
@@ -332,7 +318,7 @@ pb2_stream_kernel(StreamDev sd) {
                     tr->t_start = t_pop; tr->t_end = globaltimer_ns(); tr->smid = smid(); tr->ticket = id;
                 }
                 Retire* rec = &sd.ret[ridx & sd.ret_mask];
-                const uint32_t gen = (uint32_t)(ridx / ((unsigned long long)sd.ret_mask + 1ull)) + 1u;
+                const uint32_t gen = ring_gen(ridx, sd.ret_mask + 1ull);
                 const uint4 lo = __ldcg(reinterpret_cast<const uint4*>(&w.seen_version[(size_t)id * PB2_MAX_FLOWS]));
                 const unsigned long long res = *reinterpret_cast<volatile unsigned long long*>(&w.result[id]);
                 uint4 hi;
@@ -588,7 +574,7 @@ static int stream_cmd_slot(pb2_stream_t* s, Cmd** out) {
     return PB2_SUCCESS;
 }
 static void stream_cmd_publish(pb2_stream_t* s, Cmd* c) {
-    const uint32_t gen = (uint32_t)(s->cmd_written / (unsigned long long)s->slots) + 1u;
+    const uint32_t gen = ring_gen(s->cmd_written, s->slots);
     std::atomic_thread_fence(std::memory_order_release);
     *reinterpret_cast<volatile uint32_t*>(&c->stamp) = gen;
     s->cmd_written++;
@@ -625,15 +611,13 @@ int pb2_stream_submit(pb2_stream_t* s, const pb2_task_t* task, uint64_t cookie, 
         s->freed_head.store(h, std::memory_order_release);
         if (s->free_tickets.empty()) return PB2_ERR_OUT_OF_RESOURCE;
     }
-    // parts: ceil(widest tile / part_bytes), the rule the device applies to the slices of a tile (tile_slices)
+    // parts: the tile_parts of the widest tile, the rule the device applies to the slices of a tile
     uint32_t np = 1;
     if (s->p.part_bytes > 0 && task->body != PB2_BODY_NOP) {
         uint32_t big = 0;
         for (int f = 0; f < task->nb_flows; ++f)
             if (task->tile[f] >= 0 && s->tile_bytes[(size_t)task->tile[f]] > big) big = s->tile_bytes[(size_t)task->tile[f]];
-        np = (big + (uint32_t)s->p.part_bytes - 1) / (uint32_t)s->p.part_bytes;
-        if (np > PB2_MAX_PARTS) np = PB2_MAX_PARTS;
-        if (np < 1) np = 1;
+        np = (uint32_t)tile_parts(big, s->p.part_bytes);
     }
     {   // ready-ring capacity: entries in flight, with a view of the poll side's counter that is refreshed only when needed
         const uint64_t sub = s->sub_entries.load(std::memory_order_relaxed);
@@ -745,7 +729,7 @@ int pb2_stream_poll(pb2_stream_t* s, pb2_retire_t* out, int32_t max) {
     if (s->h_ctl->state == HS_STOPPED && s->sub_tasks.load(std::memory_order_acquire) != s->ret_tasks.load(std::memory_order_relaxed)) {
         // nobody kicked: every retire record already written is in the ring; anything else needs the kernel
         const Retire* nxt = &s->h_ret[s->ret_read & (s->slots - 1)];
-        const uint32_t g = ((uint32_t)(s->ret_read / (unsigned long long)s->slots) + 1u) & 0x7fffffffu;
+        const uint32_t g = ring_gen(s->ret_read, s->slots) & 0x7fffffffu;
         if ((*reinterpret_cast<const volatile uint32_t*>(&nxt->stamp) & 0x7fffffffu) != g) {
             int rc = stream_launch_if_parked(s);
             if (rc != PB2_SUCCESS) return rc;
@@ -754,7 +738,7 @@ int pb2_stream_poll(pb2_stream_t* s, pb2_retire_t* out, int32_t max) {
     while (n < max) {
         const Retire* rec = &s->h_ret[s->ret_read & (s->slots - 1)];
         __builtin_prefetch(&s->h_ret[(s->ret_read + 8) & (s->slots - 1)], 0, 3);
-        const uint32_t gen = ((uint32_t)(s->ret_read / (unsigned long long)s->slots) + 1u) & 0x7fffffffu;
+        const uint32_t gen = ring_gen(s->ret_read, s->slots) & 0x7fffffffu;
         const uint32_t stamp = *reinterpret_cast<const volatile uint32_t*>(&rec->stamp);
         if ((stamp & 0x7fffffffu) != gen) break;
         std::atomic_thread_fence(std::memory_order_acquire);

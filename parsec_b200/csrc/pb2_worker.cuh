@@ -25,6 +25,16 @@ struct alignas(16) TaskSmem {
     uint32_t   red[32];
 };
 
+__device__ __forceinline__ bool pushes_out(const pb2_task_t& t, int f) {
+    return t.tile[f] >= 0 && (t.access[f] & PB2_FLOW_PUSHOUT) && (t.access[f] & PB2_FLOW_ACCESS_WRITE);
+}
+
+// All threads: parsec_device_kernel_pop stage_out (device_gpu.c:2943) of a written flow to its home copy.
+__device__ __forceinline__ void pushout(Ctl* ctl, void* home, const void* dev, size_t bytes, BulkSmem* bulk = nullptr) {
+    cta_copy<false>(home, dev, bytes, bulk);
+    if (threadIdx.x == 0) atomicAdd(&ctl->bytes_d2h.v, (unsigned long long)bytes);
+}
+
 // All threads (uniform): stage in every flow whose bit is set in s.need.  One CTA-wide call per task at most.
 static __device__ __noinline__ void stage_in_needed_flows(const StageCtx c, TaskSmem* sp, BulkSmem* bulk) {
     TaskSmem& s = *sp;
@@ -39,7 +49,7 @@ static __device__ __noinline__ void stage_in_needed_flows(const StageCtx c, Task
         else {
             // slices [s0, s1) of the tile cover this part's bytes (the task may be cut differently from the tile
             // when its widest flow is another tile)
-            const uint32_t sper = ((bytes / (uint32_t)ns) + 15u) & ~15u;
+            const uint32_t sper = slice_size(bytes, ns);
             const uint32_t off = s.off[f], len = s.args.bytes[f];
             int s0 = (int)(off / sper), s1 = (int)((off + len + sper - 1) / sper);
             if (s0 > ns - 1) s0 = ns - 1;
@@ -67,10 +77,9 @@ run_task_part(const WinDev& w, TaskSmem& s, BulkSmem* bulk, int32_t id, int part
             const uint32_t v = __shfl_xor_sync(0xffffffffu, widest, o);
             widest = v > widest ? v : widest;
         }
-        const uint32_t per = ((widest / (uint32_t)nparts) + 15u) & ~15u;
-        const uint32_t off = per * (uint32_t)part < bytes ? per * (uint32_t)part : bytes;
-        const uint32_t len = (part == nparts - 1) ? bytes - off : (off + per <= bytes ? per : bytes - off);
-        const bool need = mine && (t.access[f] & PB2_FLOW_ACCESS_READ) && ld_acquire_gpu(&tile->state) != PB2_TILE_VALID;
+        uint32_t off, len;
+        slice_bounds(slice_size(widest, nparts), bytes, part, nparts, off, len);
+        const bool need = mine && needs_stage_in(tile, t.access[f]);
         const unsigned needmask = __ballot_sync(0xffffffffu, need);
         if (f < PB2_MAX_FLOWS) {
             s.args.flow[f] = mine ? reinterpret_cast<uint8_t*>(tile->dev_ptr) + off : nullptr;
@@ -97,11 +106,8 @@ run_task_part(const WinDev& w, TaskSmem& s, BulkSmem* bulk, int32_t id, int part
     // ---- pop: pushout of written flows to their home copy (parsec_device_kernel_pop stage_out) ----
 #pragma unroll
     for (int f = 0; f < PB2_MAX_FLOWS; ++f) {
-        if (f < (int)t.nb_flows && t.tile[f] >= 0 && (t.access[f] & PB2_FLOW_PUSHOUT) && (t.access[f] & PB2_FLOW_ACCESS_WRITE)) {
-            const pb2_tile_t* tile = &w.tiles[t.tile[f]];
-            cta_copy<false>(reinterpret_cast<uint8_t*>(tile->src_ptr) + s.off[f], s.args.flow[f], s.args.bytes[f], bulk);
-            if (threadIdx.x == 0) atomicAdd(&w.ctl->bytes_d2h.v, (unsigned long long)s.args.bytes[f]);
-        }
+        if (f < (int)t.nb_flows && pushes_out(t, f))
+            pushout(w.ctl, reinterpret_cast<uint8_t*>(w.tiles[t.tile[f]].src_ptr) + s.off[f], s.args.flow[f], s.args.bytes[f], bulk);
     }
     __syncthreads();
     return r;
@@ -118,14 +124,30 @@ __device__ __forceinline__ void epilog_written_flows(const WinDev& w, const pb2_
     }
 }
 
+// Thread 0 of the part that finished last, before the out-edges are released, so that the retire log is a linear
+// extension of the DAG's partial order (a successor can only retire after us).  True: the window's last task.
+__device__ __forceinline__ bool retire_task(const WinDev& w, const pb2_task_t& t, int32_t id) {
+    epilog_written_flows(w, t);
+    w.end_seq[id] = (uint32_t)atomicAdd(&w.ctl->evt.v, 1ull);
+    const uint32_t seq = (uint32_t)atomicAdd(&w.ctl->retired.v, 1ull);
+    w.retire_log[seq] = id;
+    *reinterpret_cast<volatile unsigned long long*>(&w.ctl->progress_ns.v) = globaltimer_ns();
+    return (int32_t)(seq + 1) == w.ntasks;
+}
+
 // Thread 0: store the body result of this part (CHECK bodies add their mismatch counts over the parts).
-__device__ __forceinline__ void store_result(const WinDev& w, const pb2_task_t& t, int32_t id, int part, int nparts,
-                                             unsigned long long r) {
-    if (r == ~0ull) st_relaxed_gpu(reinterpret_cast<int32_t*>(&w.ctl->done.v), kDoneBadBody);
-    if (t.body == PB2_BODY_CHECK_I32 || t.body == PB2_BODY_CHECK_F32) {
+__device__ __forceinline__ void record_result(const WinDev& w, int body, int32_t id, int part, int nparts, unsigned long long r) {
+    if (body == PB2_BODY_CHECK_I32 || body == PB2_BODY_CHECK_F32) {
         if (nparts == 1) w.result[id] = r; else if (r) atomicAdd(&w.result[id], r);
         if (r >> 32) atomicAdd(&w.ctl->body_errors.v, r >> 32);
     } else if (part == 0) w.result[id] = r;
+}
+
+// Thread 0 of a task-part worker: record_result; an unknown body id (result ~0) aborts the window.
+__device__ __forceinline__ void store_result(const WinDev& w, const pb2_task_t& t, int32_t id, int part, int nparts,
+                                             unsigned long long r) {
+    if (r == ~0ull) st_relaxed_gpu(reinterpret_cast<int32_t*>(&w.ctl->done.v), kDoneBadBody);
+    record_result(w, t.body, id, part, nparts, r);
 }
 
 }  // namespace pb2
